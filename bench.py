@@ -1,8 +1,11 @@
 #!/usr/bin/env python
 """Headline benchmark: mel-frames/sec of the Grad-TTS reverse-diffusion sampler at N=50 steps.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
+
+--dump-outputs DIR writes the mel the timed path returned in its last timed step as DIR/mel.npy (float32).  Inputs and
+weights are seeded, so two builds run with the same arguments can be compared output for output.
 
 One bench "step" = one full `Diffusion.forward(z, mask, mu, n_timesteps=50)` call on the workload
 BASELINE.json quotes the metric on (config 2: B=32 utterances x T=512 frames, fp32 in/out, per GPU;
@@ -24,6 +27,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree: leave no __pycache__ behind
 
 WORKLOADS = {
     # BASELINE.json configs[1]: Grad-TTS batch=32, T~512, N=50, fp32, 1xB200
@@ -34,6 +38,21 @@ WORKLOADS = {
 }
 FLOP_PER_FRAME_STEP = 134.15e6      # SURVEY.md 8(d): 67,077,120 MAC per mel frame per reverse step
 IDEAL_BYTES_PER_FRAME_STEP = 713280.0
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """Write each tensor of `arrays` as <out_dir>/<name>.npy in float32, DUMP_MAX_BYTES in all.  A tensor over its share
+    keeps a fixed, seeded sample of its utterances (dim 0), the same rows in every run with the same arguments."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = DUMP_MAX_BYTES // len(arrays)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        if a.nbytes > share:
+            rows = np.random.default_rng(0).choice(a.shape[0], share // (a.nbytes // a.shape[0]), replace=False)
+            a = a[np.sort(rows)]
+        np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a, dtype=np.float32))
 
 
 def load_peaks():
@@ -203,7 +222,7 @@ def cpu_reference_sample(wl, torch):
     sample = (f"{what}, PyTorch CPU fp32, {threads} threads (fastest of a sweep at this shape: {sweep} s per Euler step; "
               f"{_ncpu()} usable cores); B={b} x T={wl['T']}, {n_steps} Euler steps timed in full ({dt:.2f} s); "
               f"mel-frames/s at N={wl['N']} = B*T / (s per step * N)")
-    return frames_per_sec, sec_per_frame_step, sample, threads, kind
+    return frames_per_sec, sec_per_frame_step, sample, threads, kind, y
 
 
 def run_reference(args, wl):
@@ -213,9 +232,11 @@ def run_reference(args, wl):
         return
     vals = []
     for i in range(args.warmup + args.steps):
-        fps, spfs, sample, threads, kind = cpu_reference_sample(wl, torch)
+        fps, spfs, sample, threads, kind, y = cpu_reference_sample(wl, torch)
         if i >= args.warmup:
             vals.append((fps, spfs))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"mel": y})
     fps = statistics.median(v[0] for v in vals)
     ms_full = statistics.median(v[1] for v in vals) * wl["B"] * wl["T"] * wl["N"] * 1e3
     out = {
@@ -355,6 +376,8 @@ def run_ours(args, wl):
     eng = dec.engine()
     head = time_mode(dec, args.steps, args.warmup, sample_clocks=True)
     ms_step, value, launches, clk = head["ms_step"], head["value"], head["launches"], head["clocks"]
+    # what a caller of the timed path receives from its last step: the mel, all-gathered over the ranks when world > 1
+    head_out = (gathered.clone() if world > 1 else head["y"]) if args.dump_outputs else None
 
     # ---- end to end through the host-buffer entry point (pinned host memory in/out, copies inside the timed region)
     zh, mh, muh = z.pin_memory(), mask.pin_memory(), mu.pin_memory()
@@ -502,8 +525,10 @@ def run_ours(args, wl):
     if config5 is not None:
         out["config5"] = config5
     if cpu is not None:
-        fps_cpu, _, sample, threads, kind = cpu
+        fps_cpu, _, sample, threads, kind, _ = cpu
         out["cpu_baseline"] = {"value": fps_cpu, "unit": "mel-frames/s", "cores": threads, "kind": kind, "sample": sample}
+    if head_out is not None:
+        dump_outputs(args.dump_outputs, {"mel": head_out})
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()
@@ -527,7 +552,11 @@ def main():
     ap.add_argument("--batch", type=int, default=None, help="override B (debug only; not a valid bench line)")
     ap.add_argument("--frames", type=int, default=None, help="override T (debug only)")
     ap.add_argument("--n-timesteps", type=int, default=None, help="override N (debug only)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the mel the timed path returned in its last step as DIR/mel.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     wl = dict(WORKLOADS[args.workload])
     if args.batch: wl["B"] = args.batch
     if args.frames: wl["T"] = args.frames
